@@ -486,6 +486,30 @@ def cpu_decode_reference(model, lm, waves, gpu_hyps, seconds):
             "note": "random-init weights: top-2 margins are of the order of the bf16 logit error, see cpu_decode_reference.__doc__"}
 
 
+DUMP_SAMPLE = 1 << 20  # entries drawn from each parameter-sized buffer for --dump-outputs (4 MB each in float32)
+
+
+def step_outputs(trainer):
+    """What the last update handed its caller, copied on the device: the stats row [sample_size, ntokens, nsentences,
+    loss], the gradient norm, and the same fixed, seeded sample of the updated fp32 master weights, the gradients and
+    Adam's two moments (the full buffers are ~0.4 GB each).  Two runs of the same build agree to rounding, not bit for
+    bit: with --steps 20 --warmup 5 on a B200 (1000 W limit) they differed by 3e-5 (weights) and 1e-3 (gradients) in
+    relative Frobenius norm, so compare builds with a tolerance."""
+    flat = trainer.flat
+    idx = np.unique(np.random.RandomState(0).randint(0, flat.numel, size=DUMP_SAMPLE))
+    idx = torch.from_numpy(idx).to(flat.p32.device)
+    out = {"stats": trainer.last_stats[:4], "grad_norm": trainer._gnorm, "sample_index": idx}
+    for name, t in (("params", flat.p32), ("grads", flat.grads), ("adam_m", flat.m), ("adam_v", flat.v)):
+        out[name + "_sample"] = t.index_select(0, idx)
+    return {k: v.detach().clone() for k, v in out.items()}
+
+
+def dump_outputs(outputs, out_dir):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().double().numpy() if name == "sample_index" else t.float().cpu().numpy())
+
+
 def workload_config(n):
     return {"workload": "Conformer encoder 17x512 (ffn 2048, 8 heads, conv-k31, sinusoidal rel-pos) + CTC, V=5004, on-the-fly "
                         "fbank80+CMVN+adaptive SpecAugment from raw 16 kHz waveforms, Adam + clip 2.0, dropout 0.1",
@@ -526,6 +550,9 @@ def main():
     ap.add_argument("--sustain", type=int, default=200, help="extra timed steps after the K-step measurement (clocks settle)")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the eager-PyTorch bf16 baseline leg")
     ap.add_argument("--no-hbm-roofline", action="store_true", help="skip the per-kernel HBM roofline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the K timed steps, write what the last of them computed to DIR/<name>.npy (a fixed, seeded "
+                         "sample of the parameter-sized buffers) so that two builds can be compared")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -670,6 +697,8 @@ def main():
     l0 = lib.launch_count()
     ms, audio = timed(args.steps, False)
     launches = lib.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step_outputs(trainer), args.dump_outputs)
     timed(max(3, args.warmup), True)  # warm the host-buffer path too (copy-stream allocator pool, pinned staging)
     ms_e2e, audio_e2e = timed(args.steps, True)
     clk = clocks.stop() if rank == 0 else None

@@ -1006,6 +1006,16 @@ def pin_batching():
     out["n_cases"] = np.int64(n_cases)
     np.savez_compressed(os.path.join(GOLDEN, "batching.npz"), **out)
     print("batching: 400 random cases identical to the reference's compiled Cython packer; %d cases -> tests/golden/batching.npz" % n_cases)
+    # 100 cases at the recipe's limits (3000 frames, 24 sentences); the test redraws the inputs from the same seed
+    rs, ends = np.random.RandomState(3), {}
+    for c in range(100):
+        n = int(rs.randint(1, 200))
+        sizes = rs.randint(1, 300, size=n).astype(np.int64)
+        order = rs.permutation(n).astype(np.int64)
+        mult = int(rs.choice([1, 8]))
+        ends["c%d_ends" % c] = np.cumsum([len(b) for b in R.batch_by_size_vec(order, sizes[order], 3000, 24, mult)]).astype(np.int64)
+    np.savez_compressed(os.path.join(GOLDEN, "batching_seeded.npz"), **ends)
+    print("batching: 100 seeded cases at max_tokens 3000 / max_sentences 24 -> tests/golden/batching_seeded.npz")
 
 
 def pin_collate():
@@ -1699,7 +1709,80 @@ def pin_fullsize():
     print("full-size encoder pinned -> tests/golden/fullsize_conformer.npz")
 
 
-SECTIONS = {"global_cmvn": pin_global_cmvn, "wer_scorer": pin_wer_scorer, "lr_schedules_v2": pin_lr_schedules_v2, "scheduled_sampling": pin_scheduled_sampling, "multilevel": pin_multilevel, "lookahead": pin_lookahead, "streaming": pin_streaming, "fullsize": pin_fullsize, "text": pin_text, "lstm_lm": pin_lstm_lm, "speech_lstm": pin_speech_lstm, "dictionary": pin_dictionary, "sharding": pin_sharding, "collate": pin_collate, "batching": pin_batching, "optimizer": pin_optimizer, "beam": pin_beam, "label_smoothing": pin_label_smoothing, "frontend": pin_frontend, "ctc": pin_ctc, "conformer": pin_conformer, "encdec": pin_encdec,
+CKPT_ENC = dict(layers=1, d=32, ffn=64, heads=4, conv_channels="[8, 8, 16, 16]")  # small enough for a stored checkpoint
+
+
+def pin_checkpoint():
+    """Checkpoint interchange with the real fairseq loader, in both directions, on a small Conformer encoder.
+    (1) A checkpoint written by espresso_b200.checkpoint_utils.save_checkpoint loads through
+    fairseq.checkpoint_utils.load_checkpoint_to_cpu into the reference model, whose encoder output then equals that of the
+    same weights put in directly; the layout of that file is recorded.  (2) A checkpoint in the reference's own layout,
+    with a pickled reference config object that is not importable without fairseq, is stored for the reverse
+    direction.  -> tests/golden/checkpoint_interchange.npz, tests/golden/checkpoint_reference.pt"""
+    import tempfile
+
+    from espresso.models.transformer.speech_transformer_config import SpeechTransformerConfig as RefConfig
+    from fairseq import checkpoint_utils as RCU
+
+    from espresso_b200 import checkpoint_utils as CU
+    from espresso_b200.models import SpeechTransformerConfig, SpeechTransformerEncoderModel
+
+    c = CKPT_ENC
+    ref0 = _ref_model("conformer", **c)
+    g = torch.Generator().manual_seed(5)
+    with torch.no_grad():
+        for _, p_ in ref0.named_parameters():
+            if p_.dim() == 1:
+                p_.add_(0.1 * torch.randn(p_.shape, generator=g))
+    ref0.eval()
+
+    class _Dict:
+        def __len__(self):
+            return 50
+
+        def pad(self):
+            return 1
+
+    class _Task:
+        feat_dim, feat_in_channels, target_dictionary = 80, 1, _Dict()
+
+    cfg = SpeechTransformerConfig.from_dict(dict(
+        dropout=0.0, attention_dropout=0.0, activation_dropout=0.0, layernorm_embedding=True, max_source_positions=3600,
+        encoder=dict(embed_dim=c["d"], ffn_embed_dim=c["ffn"], layers=c["layers"], attention_heads=c["heads"],
+                     conv_channels=c["conv_channels"], normalize_before=True, learned_pos=False,
+                     relative_positional_embeddings=True, layer_type="conformer", depthwise_conv_kernel_size=31)))
+    ours = SpeechTransformerEncoderModel.build_model(cfg, _Task())
+    ours.load_state_dict(ref0.state_dict(), strict=False)
+    rs = np.random.RandomState(11)
+    feats, lens = torch.from_numpy(rs.randn(2, 41, 80).astype(np.float32)), torch.tensor([41, 30])
+    feats[1, 30:] = 0.0
+    with tempfile.TemporaryDirectory() as tmp:
+        path = os.path.join(tmp, "from_b200.pt")
+        CU.save_checkpoint(path, ours)
+        written = torch.load(path, weights_only=False)
+        rstate = RCU.load_checkpoint_to_cpu(path)
+    ref = _ref_model("conformer", **c)
+    missing, unexpected = torch.nn.Module.load_state_dict(ref, rstate["model"], strict=False)
+    assert not unexpected, unexpected
+    ref.eval()
+    with torch.no_grad():
+        out = ref(feats, lens)["encoder_out"][0]
+        out0 = ref0(feats, lens)["encoder_out"][0]
+    assert torch.equal(out, out0)
+    np.savez_compressed(os.path.join(GOLDEN, "checkpoint_interchange.npz"),
+                        file_keys=np.array(sorted(written)), model_keys=np.array(sorted(written["model"])),
+                        missing_in_reference=np.array(sorted(missing), dtype=str),
+                        optimizer_history_keys=np.array(sorted(written["optimizer_history"][-1])))
+    torch.save({"cfg": {"model": RefConfig()}, "args": None, "model": ref0.state_dict(),
+                "optimizer_history": [{"criterion_name": "CtcLossCriterion", "optimizer_name": "FP16Optimizer",
+                                       "lr_scheduler_state": {"best": None}, "num_updates": 7}],
+                "extra_state": {"train_iterator": {"epoch": 3, "iterations_in_epoch": 11}}, "last_optimizer_state": None},
+               os.path.join(GOLDEN, "checkpoint_reference.pt"))
+    print("checkpoint interchange: a b200 checkpoint loads into the reference model (same encoder output); layout -> "
+          "tests/golden/checkpoint_interchange.npz, reference-layout checkpoint -> tests/golden/checkpoint_reference.pt")
+
+
+SECTIONS = {"checkpoint": pin_checkpoint, "global_cmvn": pin_global_cmvn, "wer_scorer": pin_wer_scorer, "lr_schedules_v2": pin_lr_schedules_v2, "scheduled_sampling": pin_scheduled_sampling, "multilevel": pin_multilevel, "lookahead": pin_lookahead, "streaming": pin_streaming, "fullsize": pin_fullsize, "text": pin_text, "lstm_lm": pin_lstm_lm, "speech_lstm": pin_speech_lstm, "dictionary": pin_dictionary, "sharding": pin_sharding, "collate": pin_collate, "batching": pin_batching, "optimizer": pin_optimizer, "beam": pin_beam, "label_smoothing": pin_label_smoothing, "frontend": pin_frontend, "ctc": pin_ctc, "conformer": pin_conformer, "encdec": pin_encdec,
             "transducer": pin_transducer}
 
 

@@ -3,6 +3,7 @@ fairseq.checkpoint_utils.load_checkpoint_to_cpu into the REAL reference model (s
 reference's layout (with pickled config objects that are not importable without fairseq) loads here, and Adam's moments
 survive the round trip through fairseq's flat-fp32 optimizer layout."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -25,8 +26,6 @@ def cpu_ops(monkeypatch):
 
 
 def _ours(golden_dir):
-    import sys
-
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from test_host_orchestration import _Task, _build
 
@@ -66,7 +65,50 @@ def test_round_trip_and_optimizer_state(golden_dir, tmp_path, cpu_ops):
     assert torch.allclose(m2.flat.p32, m.flat.p32, atol=1e-6)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not mounted (GPU box)")
+def test_interchange_with_reference_fixture(golden_dir, tmp_path):
+    """Both directions against what the real reference did when the fixtures were made
+    (oracle/pin_against_reference.py::pin_checkpoint): checkpoint_reference.pt was written by the reference, with its own
+    pickled config object inside, and a file of checkpoint_interchange.npz's layout loaded through the real
+    fairseq.checkpoint_utils.load_checkpoint_to_cpu into the reference model with none of its weights missing."""
+    from espresso_b200 import checkpoint_utils as CU
+    from espresso_b200.models import SpeechTransformerConfig, SpeechTransformerEncoderModel
+
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_host_orchestration import _Task
+
+    from oracle.pin_against_reference import CKPT_ENC as c
+
+    g = np.load(os.path.join(golden_dir, "checkpoint_interchange.npz"))
+    cfg = SpeechTransformerConfig.from_dict(dict(
+        dropout=0.0, attention_dropout=0.0, activation_dropout=0.0, layernorm_embedding=True, max_source_positions=3600,
+        encoder=dict(embed_dim=c["d"], ffn_embed_dim=c["ffn"], layers=c["layers"], attention_heads=c["heads"],
+                     conv_channels=c["conv_channels"], normalize_before=True, learned_pos=False,
+                     relative_positional_embeddings=True, layer_type="conformer", depthwise_conv_kernel_size=31)))
+    # reference -> ours: the reference's layout, with a config object that only unpickles where fairseq is installed
+    state = CU.load_checkpoint_to_cpu(os.path.join(golden_dir, "checkpoint_reference.pt"))
+    assert state["optimizer_history"][-1]["num_updates"] == 7 and state["extra_state"]["train_iterator"]["epoch"] == 3
+    m = SpeechTransformerEncoderModel.build_model(cfg, _Task(50))
+    with torch.no_grad():
+        for p in m.parameters():
+            p.zero_()
+    missing, unexpected = CU.load_model_state(m, state)
+    assert not missing and not unexpected
+    for k, v in state["model"].items():
+        if k in m.state_dict() and not k.endswith("num_batches_tracked"):
+            assert torch.equal(m.state_dict()[k].float(), v.float()), k
+    # ours -> reference: the file has the layout the real loader accepted, every weight the reference model has, and
+    # the reference's own values back
+    path = str(tmp_path / "from_b200.pt")
+    CU.save_checkpoint(path, m)
+    written = torch.load(path, weights_only=False)
+    assert sorted(written) == g["file_keys"].tolist()
+    assert sorted(written["optimizer_history"][-1]) == g["optimizer_history_keys"].tolist()
+    assert sorted(written["model"]) == g["model_keys"].tolist() and g["missing_in_reference"].size == 0
+    for k, v in written["model"].items():
+        assert torch.equal(v, state["model"][k]), k
+
+
+@pytest.mark.skipif(not refshim.available(), reason="needs the reference sources (ESPRESSO_REFERENCE_ROOT)")
 def test_interchange_with_the_real_reference(golden_dir, tmp_path):
     from espresso_b200 import checkpoint_utils as CU
 

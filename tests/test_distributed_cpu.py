@@ -12,6 +12,9 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# torch threads of every rank and of the single-process reference: CPU reductions split their sums by thread count, so
+# the two sides only add in the same order with the same setting (hosts with many cores differ otherwise)
+THREADS = 2
 
 
 def _patch_ops():
@@ -44,7 +47,7 @@ def _make(golden_dir, reduce_dtype="fp32"):
 def _worker(rank, world, port, golden_dir, out_dir, reduce_dtype):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    torch.set_num_threads(2)
+    torch.set_num_threads(THREADS)
     _patch_ops()
     tr, m, samples = _make(golden_dir, reduce_dtype)
     tail = tr.train_step([samples[rank]])
@@ -75,12 +78,15 @@ def test_two_rank_update_equals_accumulated_update(golden_dir, tmp_path, reduce_
 
     from espresso_b200 import ops
     saved = {n: getattr(ops, n) for n in dir(ops)}
+    threads = torch.get_num_threads()
     try:
+        torch.set_num_threads(THREADS)
         _patch_ops()
         tr, m, samples = _make(golden_dir)
         tr.train_step(list(samples))
         ref = m.flat.p32.numpy()
     finally:
+        torch.set_num_threads(threads)
         for n, v in saved.items():
             setattr(ops, n, v)
         importlib.reload(ops)

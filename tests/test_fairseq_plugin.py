@@ -13,7 +13,7 @@ import torch
 from oracle import ops_ref, refshim
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference tree not mounted (GPU box)")
+pytestmark = pytest.mark.skipif(not refshim.available(), reason="needs the reference sources (ESPRESSO_REFERENCE_ROOT)")
 
 
 @pytest.fixture()

@@ -120,8 +120,8 @@ def test_adam_clip_and_lr_schedules_match_fairseq_fixture(golden_dir):
 
 def test_batch_packer_matches_reference_cython_fixture(golden_dir):
     """esp_batch_by_size (C ABI, host code) vs the batches produced by the reference's compiled Cython packer
-    (fairseq/data/data_utils_fast.pyx) recorded in tests/golden/batching.npz; and live against oracle/_ref when the
-    compiled reference is present."""
+    (fairseq/data/data_utils_fast.pyx) recorded in tests/golden/batching.npz, and at the recipe's limits on the seeded
+    cases recorded in tests/golden/batching_seeded.npz."""
     from espresso_b200.data import batching as Bt
 
     g = np.load(os.path.join(golden_dir, "batching.npz"))
@@ -137,21 +137,16 @@ def test_batch_packer_matches_reference_cython_fixture(golden_dir):
         raise RuntimeError("oversized sample must be rejected")
     except AssertionError:
         pass
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-    import glob
-    import sys
-    if glob.glob(os.path.join(ref_dir, "data_utils_fast*.so")):
-        sys.path.insert(0, ref_dir)
-        import data_utils_fast as R
-        rs = np.random.RandomState(3)
-        for _ in range(100):
-            n = int(rs.randint(1, 200))
-            sizes = rs.randint(1, 300, size=n).astype(np.int64)
-            order = rs.permutation(n).astype(np.int64)
-            mult = int(rs.choice([1, 8]))
-            ref = R.batch_by_size_vec(order, sizes[order], 3000, 24, mult)
-            got = Bt.batch_by_size(order, sizes, 3000, 24, mult)
-            assert len(ref) == len(got) and all(np.array_equal(a, b) for a, b in zip(ref, got))
+    ref = np.load(os.path.join(golden_dir, "batching_seeded.npz"))
+    rs = np.random.RandomState(3)
+    for c in range(100):
+        n = int(rs.randint(1, 200))
+        sizes = rs.randint(1, 300, size=n).astype(np.int64)
+        order = rs.permutation(n).astype(np.int64)
+        mult = int(rs.choice([1, 8]))
+        got = Bt.batch_by_size(order, sizes, 3000, 24, mult)
+        assert np.array_equal(np.cumsum([len(b) for b in got]), ref["c%d_ends" % c]), c
+        assert np.array_equal(np.concatenate(got), order)
 
 
 def test_collate_matches_reference_fixture(golden_dir):
